@@ -3,7 +3,7 @@
 backward, on synthetic batches of the reference's shapes.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|reference-cuda]
-                    [--config D|B|C|E] [--scaling weak|strong]
+                    [--config D|B|C|E] [--scaling weak|strong] [--dump-outputs DIR]
 
 Configs (BASELINE.json `configs`, SURVEY.md section 8d):
   D (default, the metric of record)  Atari PPO: gae -> ppo_error, T=128, B=4096, N=6 per GPU (`--scaling strong`: B=4096 in
@@ -54,6 +54,7 @@ NSETS = 4
 # Atari VAC of pong_ppo_config.py:21-28 (obs [4,84,84], encoder [64,64,128] k8s4/k4s2/k3s1, fc 6272->128, actor 128->128->6,
 # critic 128->128->1): 16448 + 65600 + 73856 + 802944 + 17286 + 16641 parameters
 VAC_PARAMS = 992775
+DUMP_LIMIT = 64 << 20  # --dump-outputs: bytes written at most (the largest config, P, writes 22 MiB)
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -220,6 +221,12 @@ class DeviceStepD:
     def loss_vector(self):
         return self.out
 
+    def outputs(self):
+        """what a caller of gae_ppo_error receives from this step: the advantage, ppo_loss, ppo_info and the gradients"""
+        names = ('policy_loss', 'value_loss', 'entropy_loss', 'kl_div', 'approx_kl', 'clipfrac')
+        return dict(adv=self.adv, **{n: self.out[i] for i, n in enumerate(names)}, grad_logit_new=self.grad_logit,
+                    grad_value_new=self.grad_value)
+
     def __call__(self):
         for _, k in self.kernels():
             k()
@@ -320,6 +327,9 @@ class DeviceStepP(DeviceStepD):
 
     def launches_per_step(self):
         return 5  # gae scan, returns + both statistics, ppo forward-with-gradient, finalize_sums, backward check
+
+    def outputs(self):
+        return dict(super().outputs(), value=self.vout, return_=self.rout, unnormalized_return=self.unnorm)
 
     def check(self, host_batch):
         from oracle import rl_oracle
@@ -477,6 +487,10 @@ class DeviceStepTD:
     def loss_vector(self):
         return self.loss
 
+    def outputs(self):
+        grad = 'grad_q' if self.wl.key == 'B' else 'grad_dist'
+        return {'loss': self.loss, 'td_error_per_sample': self.td, grad: self.grad}
+
     def __call__(self):
         for _, k in self.kernels():
             k()
@@ -565,6 +579,10 @@ class DeviceStepE:
 
     def loss_vector(self):
         return self.out
+
+    def outputs(self):
+        return dict(policy_loss=self.out[0], value_loss=self.out[1], entropy_loss=self.out[2],
+                    grad_target_output=self.grad_logit, grad_value=self.grad_value)
 
     def __call__(self):
         for _, k in self.kernels():
@@ -938,6 +956,8 @@ def run_gpu(args):
         h1.record(main)
         barrier()
         dbg('timed replay done')
+        # device-side copy of the last timed step's outputs before later replays reuse its buffer set
+        last_outputs = {k: v.clone() for k, v in sets[(K - 1) % NSETS].outputs().items()} if args.dump_outputs else None
         dev_ms = e0.elapsed_time(e1)
         host_ms = h0.elapsed_time(h1)
         # keep the GPU under the same load while nvidia-smi samples (a 20-step region lasts 0.3 ms)
@@ -1142,6 +1162,8 @@ def run_gpu(args):
             line['param_allreduce'] = dict(par, ms_per_step_with=par_ms,
                                            note='the step followed by an NCCL all-reduce of a %d-float dummy gradient '
                                                 'bucket (Atari VAC net) on the same stream, eager launches' % VAC_PARAMS)
+        if last_outputs is not None:
+            dump_outputs(args.dump_outputs, last_outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         # graphs that captured NCCL work must be gone before the communicator is torn down; then leave without waiting on
@@ -1153,6 +1175,18 @@ def run_gpu(args):
         sys.stdout.flush()
         sys.stderr.flush()
         os._exit(0)
+
+
+def dump_outputs(out_dir, tensors):
+    """DIR/<name>.npy in float32 for every output of the last timed step (rank 0's shard under data parallelism)"""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in tensors.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit('--dump-outputs: %d bytes of outputs exceed %d' % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
 
 
 def run_reference(args):
@@ -1234,6 +1268,9 @@ def main():
                     help='e2e: int64 actions / fp32 flags on the wire (default: one byte each, widened on the device)')
     ap.add_argument('--e2e-separate-copies', action='store_true',
                     help='e2e: one pinned tensor and one H2D copy per input (default: di_engine_b200.PackedBatch, one copy)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps write the outputs of the last one (losses, advantages, gradients) as '
+                         'DIR/<name>.npy, float32; the inputs are seeded, so two builds can be compared output for output')
     args = ap.parse_args()
     if args.impl == 'reference':
         run_reference(args)

@@ -9,9 +9,11 @@
 * ``install()`` / ``uninstall()`` rebinding and the ``hpc_rll`` shim layout (ding/hpc_rl/wrapper.py:62-73);
 * the product refuses to run without CUDA (no CPU fallback) and never imports the oracle.
 """
+import collections
 import contextlib
 import ctypes
 import inspect
+import json
 import os
 import re
 import sys
@@ -23,7 +25,7 @@ import torch.nn as nn
 
 import di_engine_b200 as b2
 from di_engine_b200 import _lib, ops
-from tests import cases
+from tests import cases, golden_io
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -120,26 +122,30 @@ def test_signatures_match_reference_defaults():
                                 ('bootstrap_values', E), ('mask', None)]
 
 
+def _reference_api():
+    with open(os.path.join(golden_io.GOLDEN_DIR, 'reference', 'api.json')) as f:
+        return json.load(f)
+
+
 def test_every_hot_path_signature_matches_the_live_reference():
-    """every rebound function, against the unmodified reference: same parameter names in the same order, same defaults
-    (callables / modules by type or by name)"""
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip('reference not importable here')
-    ref = ref_loader.load()
+    """every rebound function, against the unmodified reference (its signatures recorded in tests/golden/reference/api.json):
+    same parameter names in the same order, same defaults (callables / modules by type or by name)"""
+    ref = _reference_api()
     for name in b2.rl_utils.HOT_PATH_FUNCTIONS:
-        ours, theirs = getattr(b2.rl_utils, name), getattr(ref, name, None)
+        ours, theirs = getattr(b2.rl_utils, name), ref['functions'].get(name)
         assert theirs is not None, name
-        po, pt = inspect.signature(ours).parameters, inspect.signature(theirs).parameters
-        assert list(po) == list(pt), (name, list(po), list(pt))
+        po, pt = inspect.signature(ours).parameters, dict(theirs['params'])
+        assert list(po) == [k for k, _ in theirs['params']], (name, list(po), list(pt))
         for k in po:
-            a, b = po[k].default, pt[k].default
-            if callable(a) or callable(b):
-                assert type(a) is type(b) or getattr(a, '__name__', None) == getattr(b, '__name__', None), (name, k)
+            a, b = po[k].default, pt[k]
+            if a is inspect.Parameter.empty or 'empty' in b:
+                assert a is inspect.Parameter.empty and 'empty' in b, (name, k)
+            elif callable(a) or 'type' in b:
+                assert type(a).__name__ == b.get('type') or getattr(a, '__name__', None) == b.get('name'), (name, k)
             else:
-                assert a == b, (name, k, a, b)
+                assert json.loads(json.dumps(a)) == b['value'], (name, k, a, b)
     for name in b2.rl_utils.HOT_PATH_TYPES:
-        assert getattr(b2.rl_utils, name)._fields == getattr(ref, name)._fields, name
+        assert list(getattr(b2.rl_utils, name)._fields) == ref['types'][name], name
 
 
 def test_shape_fns():
@@ -160,8 +166,9 @@ def test_shape_fns():
     assert tuple(r.shape_fn_vtrace_discrete_action([d], {})) == (4, 8, 16)
 
 
-def test_no_cpu_fallback_and_no_oracle_import():
-    assert not torch.cuda.is_available(), "this test documents the CPU-only container"
+def test_no_cpu_fallback_and_no_oracle_import(monkeypatch):
+    """without a CUDA device every operator raises (simulated, so that the check also runs on a machine with a GPU)"""
+    monkeypatch.setattr(torch.cuda, 'is_available', lambda: False)
     t = torch.zeros(4, 3)
     with pytest.raises(_lib.B200RLError):
         b2.gae(b2.gae_data(t, t.clone(), t, None, None))
@@ -378,15 +385,34 @@ def test_install_rebinds_and_uninstall_restores(dry, monkeypatch):
     assert fake['ding.policy.ppo'].gae is ref_gae and fake['ding.rl_utils'].ppo_error is ref_ppo
 
 
-def test_install_on_the_live_reference_rebinds_every_hot_path_function(dry):
-    """the real ding.rl_utils modules (oracle/ref_loader.py): install() replaces every function of HOT_PATH_FUNCTIONS in the
-    package namespace and in the submodule that defines it; a policy-like module that imported the names keeps working through
-    the rebinding; uninstall() restores the originals"""
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip('reference not importable here')
-    ref = ref_loader.load()
-    originals = {n: getattr(ref, n) for n in b2.rl_utils.HOT_PATH_FUNCTIONS}
+def test_install_on_the_live_reference_rebinds_every_hot_path_function(dry, monkeypatch):
+    """the module layout of the real ding.rl_utils (recorded in tests/golden/reference/api.json: which submodule defines each
+    function, which submodules hold it): install() replaces every function of HOT_PATH_FUNCTIONS in the package namespace
+    and in the submodule that defines it; a policy-like module that imported the names keeps working through the
+    rebinding; uninstall() restores the originals"""
+    api = _reference_api()
+    pkg = types.ModuleType('ding.rl_utils')
+    mods = {'ding': types.ModuleType('ding'), 'ding.rl_utils': pkg}
+    for m in api['modules']:
+        mods[m] = types.ModuleType(m)
+    for name, mod in mods.items():
+        monkeypatch.setitem(sys.modules, name, mod)
+
+    def stand_in(name, module):
+        def fn(*a, **k):
+            return 'reference'
+        fn.__name__, fn.__module__ = name, module
+        return fn
+
+    originals = {n: stand_in(n, api['functions'][n]['module']) for n in b2.rl_utils.HOT_PATH_FUNCTIONS}
+    for n, fn in originals.items():
+        setattr(pkg, n, fn)
+    for m, held in api['modules'].items():
+        for n in held:
+            setattr(mods[m], n, originals[n])
+    for n, fields in api['types'].items():
+        setattr(pkg, n, collections.namedtuple(n, fields))
+    ref = pkg
     policy = types.ModuleType('ding.policy.fake_for_install_test')
     for n, fn in originals.items():
         setattr(policy, n, fn)  # `from ding.rl_utils import ...` at import time
@@ -516,6 +542,75 @@ def test_live_hpc_wrapper_dispatches_into_the_shim(dry, monkeypatch):
         assert len(hw.hpc_fns['gae']) == 3 and 'gae_%d_%d' % (T, B) not in hw.hpc_fns['gae']
     finally:
         hw.hpc_fns.clear()
+        for k in list(sys.modules):
+            if k == 'hpc_rll' or k.startswith('hpc_rll.'):
+                del sys.modules[k]
+
+
+def hpc_wrapper_calls(api):
+    """(operator, data, positional, keyword arguments): the calls of the test above, through ``api``'s namedtuples"""
+    g = torch.Generator().manual_seed(5)
+    T, B = 16, 8
+    d = api.gae_data(torch.randn(T, B, generator=g), torch.randn(T, B, generator=g), torch.randn(T, B, generator=g),
+                     torch.zeros(T, B), None)
+    yield 'gae', d, (0.99, 0.95), {}
+    yield 'gae', d, (), {'gamma': 0.9, 'lambda_': 0.8}
+    op, t, p = cases.ppo_case(3, 12, 5, weight='tensor')
+    tt = cases.prepare(op, t)
+    yield 'ppo_error', api.ppo_data(*[tt[k] for k in ('logit_new', 'logit_old', 'action', 'value_new', 'value_old', 'adv',
+                                                      'return_', 'weight', 'logit_pretrained')]), (0.2, True, None), {}
+    op, t, p = cases.qntd_case(4, 8, 4, 3)
+    yield 'q_nstep_td_error', api.q_nstep_td_data(*[t[k] for k in ('q', 'next_n_q', 'action', 'next_n_action', 'reward',
+                                                                   'done', 'weight')]), (0.95, ), {'nstep': 3}
+    op, t, p = cases.dntd_case(5, 6, 3, 51, 2)
+    yield 'dist_nstep_td_error', api.dist_nstep_td_data(*[t[k] for k in ('dist', 'next_n_dist', 'act', 'next_n_act', 'reward',
+                                                                         'done', 'weight')]), (0.95, -10., 10., 51, 2), {}
+    op, t, p = cases.td_lambda_case(6, 8, 4)
+    yield 'td_lambda_error', api.td_lambda_data(t['value'], t['reward'], t['weight']), (0.9, 0.8), {}
+    op, t, p = cases.vtrace_case(7, 4, 8, 6)
+    yield 'vtrace_error_discrete_action', api.vtrace_data(*[t[k] for k in ('target_output', 'behaviour_output', 'action',
+                                                                           'value', 'reward', 'weight')]), (0.99, 0.95), {}
+    for Tn in (3, 4, 5, 6):
+        yield 'gae', api.gae_data(torch.zeros(Tn, 2), torch.zeros(Tn, 2), torch.zeros(Tn, 2), None, None), (), {}
+
+
+HPC_SHAPE_FN = {'gae': 'shape_fn_gae', 'ppo_error': 'shape_fn_ppo', 'q_nstep_td_error': 'shape_fn_qntd',
+                'dist_nstep_td_error': 'shape_fn_dntd', 'td_lambda_error': 'shape_fn_td_lambda',
+                'vtrace_error_discrete_action': 'shape_fn_vtrace_discrete_action'}
+HPC_FIRST_CALLS = {'gae': ['b200rl_gae'], 'ppo_error': ['b200rl_ppo_fused_supported', 'b200rl_ppo_fwd_grad'],
+                   'q_nstep_td_error': ['b200rl_qntd_fwd'], 'dist_nstep_td_error': ['b200rl_dntd_fwd'],
+                   'td_lambda_error': ['b200rl_td_lambda_fwd'],
+                   'vtrace_error_discrete_action': ['b200rl_vtrace_fused_supported', 'b200rl_vtrace_fwd_grad']}
+
+
+def test_recorded_hpc_wrapper_dispatch_reaches_the_c_abi(dry, monkeypatch):
+    """What the reference's decorator (ding/hpc_rl/wrapper.py:86-133) with ``ding.enable_hpc_rl = True`` hands to
+    ``hpc_rll`` for each call of ``hpc_wrapper_calls``, recorded from the live reference in
+    tests/golden/reference/hpc_dispatch.json: the module and class it imports, the shape it constructs them with (which
+    this package's ``shape_fn_*`` must reproduce) and the arguments it keeps.  Replayed against the classes
+    ``install_hpc_rll()`` registers, every call must reach the C ABI (here: the recording stand-in for the library)."""
+    import importlib
+    with open(os.path.join(golden_io.GOLDEN_DIR, 'reference', 'hpc_dispatch.json')) as f:
+        recorded = json.load(f)
+    for k in list(sys.modules):
+        if k == 'hpc_rll' or k.startswith('hpc_rll.'):
+            monkeypatch.delitem(sys.modules, k)
+    b2.install_hpc_rll(force=True)
+    calls = list(hpc_wrapper_calls(b2.rl_utils))
+    assert len(calls) == len(recorded)
+    try:
+        for (fn, data, args, kwargs), r in zip(calls, recorded):
+            assert r['fn'] == fn
+            assert list(getattr(b2.rl_utils, HPC_SHAPE_FN[fn])((data, ) + tuple(args), kwargs)) == r['shape'], fn
+
+            def arg(x):
+                return data[x['field']] if 'field' in x else x.get('value')
+
+            dry.calls.clear()
+            op = getattr(importlib.import_module(r['module']), r['cls'])(*r['shape']).cuda()
+            op(*[arg(x) for x in r['args']], **{k: arg(v) for k, v in r['kwargs'].items()})
+            assert dry.calls[:len(HPC_FIRST_CALLS[fn])] == HPC_FIRST_CALLS[fn], (fn, dry.calls)
+    finally:
         for k in list(sys.modules):
             if k == 'hpc_rll' or k.startswith('hpc_rll.'):
                 del sys.modules[k]

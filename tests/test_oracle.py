@@ -1,19 +1,23 @@
 """CPU suite (-m "not gpu"): pins the oracle restatement.
 
 1. against the committed golden fixtures (outputs of the unmodified reference, see tests/golden/make_golden.py);
-2. against the live reference when /root/reference is present (build container only) -- bit-exact, since the
-   oracle uses the same torch primitives in the same order;
+2. against what the unmodified reference computed, bit-exact, since the oracle uses the same torch primitives in the
+   same order (the fixtures, and ``tests/golden/reference/`` for the medium shapes and the policy-level lines);
 3. relational identities the reference's own tests hold (tests/test_td.py:113-126, :196-204,
    tests/test_value_rescale.py:21-26).
 """
+import os
+
 import numpy as np
 import pytest
 import torch
 
-from oracle import ref_loader, rl_oracle
+from oracle import rl_oracle
 from tests import cases, golden_io
+from tests.golden import make_golden
 
 CASES = cases.build_cases()
+REF_DIR = os.path.join(golden_io.GOLDEN_DIR, 'reference')
 
 
 def test_fixture_set_matches_case_registry():
@@ -45,32 +49,36 @@ def test_case_builders_reproduce_fixture_inputs(name):
             assert torch.equal(v, tensors[k]), k
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='reference tree only exists in the build container')
 @pytest.mark.parametrize('name', sorted(CASES.keys()))
 def test_oracle_bit_exact_vs_live_reference(name):
+    """bit for bit against the reference's outputs stored in the fixture (single-threaded on both sides)"""
     op, tensors, params = CASES[name]
     torch.set_num_threads(1)
-    ref = ref_loader.load()
-    want = cases.run_api(ref, op, tensors, params)
+    want = golden_io.load(name)[3]
     got = cases.run_oracle(rl_oracle, op, tensors, params)
     cases.compare(got, want, exact=True)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='reference tree only exists in the build container')
 def test_oracle_vs_live_reference_bench_shapes():
-    """Medium shapes of the five BASELINE configs (kept to a few seconds)."""
-    ref = ref_loader.load()
-    big = {
-        'gae_D': cases.gae_case(100, 128, 512, p_done=0.01),
-        'ppo_D': cases.ppo_case(101, 128 * 64, 6, clip_ratio=0.2),
-        'qntd_B': cases.qntd_case(102, 512, 6, 3, value_gamma='tensor', gamma=0.99, done='bern'),
-        'dntd_C': cases.dntd_case(103, 512, 6, 51, 3, gamma=0.99, value_gamma='tensor'),
-        'vtrace_E': cases.vtrace_case(104, 64, 256, 6, gamma=0.99, lambda_=0.95),
-    }
-    for name, (op, tensors, params) in big.items():
-        want = cases.run_api(ref, op, tensors, params)
+    """Medium shapes of the five BASELINE configs (kept to a few seconds), against the reference's outputs stored in
+    tests/golden/reference/bench_shapes.npz: small outputs whole, large ones as a fixed sample plus their sums."""
+    with np.load(os.path.join(REF_DIR, 'bench_shapes.npz')) as z:
+        want = {k: z[k] for k in z.files}
+    for name, (op, tensors, params) in make_golden.bench_shape_cases().items():
         got = cases.run_oracle(rl_oracle, op, tensors, params)
-        cases.compare(got, want, rtol=1e-6, atol=1e-6)
+        keys = {k.split('/')[1] for k in want if k.startswith(name + '/')}
+        assert keys == set(got), (name, keys, set(got))
+        for k in sorted(keys):
+            a, w = np.asarray(got[k]), name + '/' + k
+            if w in want:
+                assert np.allclose(a, want[w], rtol=1e-6, atol=1e-6), (w, float(np.max(np.abs(a - want[w]))))
+                continue
+            assert a.shape == tuple(want[w + '/shape']), w
+            flat = a.reshape(-1)
+            sample = flat[make_golden.sample_index(flat.size)]
+            assert np.allclose(sample, want[w + '/sample'], rtol=1e-6, atol=1e-6), (w, float(np.max(np.abs(sample - want[w + '/sample']))))
+            total, abs_total = want[w + '/sums']
+            assert abs(flat.astype(np.float64).sum() - total) <= 1e-6 * abs_total + 1e-6, w
 
 
 def test_nstep1_equals_one_step_form():
@@ -120,25 +128,18 @@ def test_projection_conserves_mass():
     assert torch.allclose(per, torch.full_like(per, float(np.log(51.0))), atol=1e-5)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='reference not importable here')
 def test_policy_level_restatements_match_the_reference_lines():
     """ding/policy/ppo.py cannot be imported (it pulls the whole framework), so its lines :276-292 and :304-306 are executed
-    here literally around the LIVE reference gae and compared with the oracle's restatement, bit for bit."""
-    ref = ref_loader.load()
-    g = torch.Generator().manual_seed(77)
-    for shape, std in (((400, ), None), ((400, ), 1.7320508), ((33, 5), 0.6)):
-        value = torch.randn(*shape, generator=g)
-        next_value = torch.randn(*shape, generator=g)
-        reward = torch.randn(*shape, generator=g)
-        done = (torch.rand(*shape, generator=g) < 0.05).float()
-        traj = done.clone()
-        traj[-1] = 1.0
+    here literally around the reference gae (its outputs on these inputs are stored in tests/golden/reference/policy_gae.npz)
+    and compared with the oracle's restatement, bit for bit."""
+    inputs, g = make_golden.policy_gae_inputs()
+    with np.load(os.path.join(REF_DIR, 'policy_gae.npz')) as z:
+        ref_adv = [torch.from_numpy(z['adv_%d' % i]) for i in range(len(inputs))]
+    for (value, next_value, reward, done, traj, std), adv in zip(inputs, ref_adv):
         got = rl_oracle.ppo_policy_gae_returns(value, next_value, reward, done, traj, 0.99, 0.95, std)
-        v, nv = value.clone(), next_value.clone()
+        v = value.clone()
         if std is not None:
             v *= std
-            nv *= std
-        adv = ref.gae(ref.gae_data(v, nv, reward, done, traj), 0.99, 0.95)
         unnormalized_returns = v + adv
         if std is not None:
             val, ret = v / std, unnormalized_returns / std

@@ -4,8 +4,11 @@
               archive oracle/_ref/ding_hotpath.zip elsewhere) on CPU tensors -- proves the port is a faithful harness;
   b200_dry    ``di_engine_b200.rl_utils`` on CPU with a recording stand-in for the CUDA library: shapes, autograd wiring,
               error behaviour and the host-side shape algebra, no GPU needed (values are uninitialised memory);
-  b200        ``di_engine_b200.rl_utils`` on the GPU (``-m gpu``): every assertion of the reference's test AND, whenever the
-              reference is importable next to the GPU, value parity of every output and gradient against it (1e-5).
+  b200        ``di_engine_b200.rl_utils`` on the GPU (``-m gpu``): every assertion of the reference's test AND value parity
+              of every output and gradient against what the reference recorded on the same inputs (1e-5).
+
+What the reference records is stored in ``tests/golden/reference/suite_records.npz`` (tests/golden/make_golden.py), so
+the parity check needs no reference next to the GPU; the ``reference`` run checks those records against the reference.
 
 Ported from ding/rl_utils/tests/test_gae.py, test_ppo.py (discrete, continuous, shape_fn), test_a2c.py (discrete), test_td.py (the operators on this
 path: q_nstep, q_nstep_ngu, bdq_nstep, q_1step_compatible, dist_1step, dist_1step_compatible, dist_1step multi agent,
@@ -14,6 +17,9 @@ tests), test_vtrace.py (discrete), test_happo.py (discrete), test_retrace.py, te
 ports seed them (so the three implementations see identical bits) and keep every assertion.
 """
 import contextlib
+import functools
+import json
+import os
 
 import numpy as np
 import pytest
@@ -22,8 +28,10 @@ import torch
 import di_engine_b200 as b2
 from di_engine_b200 import _lib, ops
 from oracle import ref_loader
+from tests import golden_io
 
 HAVE_REF = ref_loader.available()
+RECORDS = os.path.join(golden_io.GOLDEN_DIR, 'reference', 'suite_records.npz')
 IMPLS = [
     pytest.param('reference', marks=pytest.mark.skipif(not HAVE_REF, reason='reference not importable here')),
     pytest.param('b200_dry'),
@@ -87,14 +95,30 @@ def _gen(seed):
     return torch.Generator().manual_seed(seed)
 
 
+def record_key(body, args):
+    """name of one run of a ported test body in the stored reference records"""
+    return body.__qualname__ + repr(tuple(args))
+
+
+@functools.lru_cache(maxsize=None)
+def _reference_records():
+    with np.load(RECORDS) as z:
+        values, index = z['values'], json.loads(bytes(z['index']).decode())
+    out = {}
+    for name, at, shape in index:
+        key, k = name.rsplit('::', 1)
+        out.setdefault(key, {})[k] = values[at:at + int(np.prod(shape))].astype(np.float64).reshape(shape)
+    return out
+
+
 def _run(body, impl, *args):
-    """Run a ported test body on ``impl``; on the GPU also run it on the reference and compare every recorded value."""
+    """Run a ported test body on ``impl``; on the GPU and on the reference compare every recorded value with what the
+    reference recorded on the same inputs."""
     api, dev, kind = impl
     rec = Rec()
     body(api, dev, rec, *args)
-    if kind == 'b200' and HAVE_REF:
-        want = Rec()
-        body(ref_loader.load(), 'cpu', want, *args)
+    if kind in ('b200', 'reference'):
+        want = _reference_records()[record_key(body, args)]
         assert set(rec) == set(want)
         for k in want:
             a, b = rec[k], want[k]
@@ -459,6 +483,7 @@ def _quantile_body(kind):
             assert td_error_per_sample.shape == (batch_size, )
             rec.put('vg_loss_%d' % nstep, loss)
 
+    body.__qualname__ = '_quantile_body(%r)' % kind
     return body
 
 
